@@ -13,9 +13,11 @@ distribution + mean/frequency/entropy; weak scaling) and carries, next to it:
   python bench.py [--gpus N] [--steps K] [--warmup W]                 # this framework
   python bench.py --workload C4                                       # the ABC line on its own
   python bench.py --impl reference [--gpus N] --steps K --warmup W    # CPU restatement, all host cores
+  python bench.py --dump-outputs DIR                                  # + the last timed step's results as DIR/*.npy
 
 Every step simulates a different index range, so nothing is reused; a 256 MiB buffer is rewritten
-before every step (L2 flush).
+before every step (L2 flush).  The index ranges and seeds depend on the arguments only, so two builds run
+with the same arguments can be compared output for output with --dump-outputs.
 """
 import argparse
 import json
@@ -43,6 +45,7 @@ WANT = ("stop_reason", "nminus", "nplus", "time", "n_events", "kmax", "mean", "f
         "hist")
 ABC_THRESHOLDS = (0.05, 0.1, 0.1, 0.1)
 ABC_BINS = 256
+DUMP_BYTES = 64_000_000  # --dump-outputs: all files together, .npy headers included
 
 
 def parse():
@@ -64,6 +67,8 @@ def parse():
     ap.add_argument("--no-strong", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step as DIR/<name>.npy (at most 64 MB)")
     return ap.parse_args()
 
 
@@ -179,11 +184,13 @@ def cpu_abc(m, ob, o, oo, seconds, cores, draws=None):
         t1 = max(time.perf_counter() - t0, 1e-3)
         draws = int(max(1000, min(200_000, probe * seconds / t1)))
     rates = abc_priors_numpy(draws)
+    idx0 = 20_000_000
     t0 = time.perf_counter()
-    r = ob.abc_batch(oo, 20_000_000, draws, rates, target, ABC_THRESHOLDS, cores)
+    r = ob.abc_batch(oo, idx0, draws, rates, target, ABC_THRESHOLDS, cores)
     dt = time.perf_counter() - t0
     return {"events": int(r.total_events), "seconds": dt, "replicates": draws, "cores": cores,
-            "events_per_sec": r.total_events / dt, "sims_per_sec": draws / dt, "accepted": int(r.accept.sum())}
+            "events_per_sec": r.total_events / dt, "sims_per_sec": draws / dt, "accepted": int(r.accept.sum()),
+            "batch": r, "rates": rates, "first_index": idx0}
 
 
 def reference_arm(args, rank, world):
@@ -214,7 +221,8 @@ def reference_arm(args, rank, world):
         def step(i):
             t0 = time.perf_counter()
             r = ob.run_batch(oo, o.idx_begin + i * n, n, cores)
-            return {"events": int(r.total_events), "seconds": time.perf_counter() - t0}
+            return {"events": int(r.total_events), "seconds": time.perf_counter() - t0, "batch": r,
+                    "first_index": o.idx_begin + i * n}
     for w in range(args.warmup):
         step(w)
     events, tot_t = 0, 0.0
@@ -222,6 +230,13 @@ def reference_arm(args, rank, world):
         r = step(args.warmup + s)
         tot_t += r["seconds"]
         events += r["events"]
+    if args.dump_outputs:
+        b = r["batch"]
+        cols = ("distance", "accept", "n_events", "stop") if abc else ("stop", "nminus", "nplus", "time", "n_events")
+        rows = {c: (getattr(b, c), getattr(b, c).dtype) for c in cols}
+        if abc:
+            rows["prior_rates"] = (r["rates"], np.float32)
+        dump_outputs(args.dump_outputs, rows, r["first_index"])
     metric, unit = ("abc_sims_per_sec", "sims/s") if abc else ("ssa_events_per_sec", "events/s")
     v = (n * args.steps / tot_t) if abc else events / tot_t
     sample = (f"{n} {'prior draws' if abc else 'replicates'} of {args.workload} per step over {cores} host threads "
@@ -310,6 +325,44 @@ def gather_floats(e, x):
     return [float(p.item()) for p in parts]
 
 
+def dump_outputs(d, rows, first_index, extra=None, rank=0, world=1):
+    """--dump-outputs: result columns as DIR/<name>.npy, floats as float32, integers as float64 (exact below 2**53).
+    `rows` maps a name to (tensor or array, numpy dtype of its elements); row i of every column belongs to
+    replicate (or prior draw) first_index + i, and replicate_index.npy holds that index for each row written.
+    Columns that would exceed DUMP_BYTES together are cut to the same fixed, seeded sample of rows, in index
+    order.  `extra` (host arrays written whole) counts against the same budget.  With several ranks, rank r
+    writes DIR/rank<r>/."""
+    if world > 1:
+        d = os.path.join(d, f"rank{rank}")
+    os.makedirs(d, exist_ok=True)
+    extra = {k: np.asarray(v) for k, v in (extra or {}).items()}
+    extra = {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float64) for k, v in extra.items()}
+    n = len(next(iter(rows.values()))[0])
+
+    def row_bytes(x, dtype):
+        return int(np.prod(x.shape[1:], dtype=np.int64)) * (4 if np.dtype(dtype) == np.float32 else 8)
+    per_row = 8 + sum(row_bytes(x, dt) for x, dt in rows.values())
+    budget = DUMP_BYTES - sum(v.nbytes for v in extra.values()) - 4096 * (len(rows) + len(extra) + 1)  # headers
+    keep = np.arange(n)
+    if per_row * n > budget:
+        keep = np.sort(np.random.default_rng(0).choice(n, max(budget // per_row, 1), replace=False))
+    out = dict(extra, replicate_index=(first_index + keep).astype(np.float64))
+    for name, (x, dtype) in rows.items():
+        if hasattr(x, "index_select"):  # a torch tensor: sample on its device, then copy
+            import torch
+            x = x.index_select(0, torch.from_numpy(keep).to(x.device)).cpu().numpy()
+        else:
+            x = np.asarray(x)[keep]
+        x = x.view(dtype)
+        out[name] = x if x.dtype in (np.float32, np.float64) else x.astype(np.float64)
+    for name, x in out.items():
+        np.save(os.path.join(d, name + ".npy"), x)
+
+
+def result_dtypes(m):
+    return {name: dtype for name, dtype, _ in m.RESULT_FIELDS}
+
+
 def oracle_check(e, opts, tensors, idx0, picks, dyn=None):
     """Replicates of the batch that was just timed against the CPU oracle (the specification of the native
     stream), bit for bit: stop reason, counts, events, f32 clock bits, final distribution.  Outside the timed
@@ -390,6 +443,7 @@ def ssa_leg(e, args, workload, reps, steps, warmup, idx_base, check=0, sample_cl
     out.value = out.events_all / (out.ms_all * 1e-3)
     out.events, out.alg_bytes, out.kernel_ms, out.steps = events, alg_bytes, float(np.mean(kernel_ms)), steps
     out.opts, out.knobs, out.want, out.desc, out.reps = opts, knobs, want, desc, reps
+    out.tensors, out.last_idx0 = tensors, last_idx0
     out.kmax = int(tensors["kmax"].max().item())
     # ---- what was simulated, outside the timed region: invariants on every replicate of the last step ... ----
     stops = tensors["stop_reason"].cpu().numpy() & 0xFF
@@ -478,13 +532,14 @@ def roofline_block(leg, workload, clocks):
     return r
 
 
-def abc_leg(e, args, draws_total, with_cpu, with_e2e):
+def abc_leg(e, args, draws_total, with_cpu, with_e2e, steps=1, warmup=3, dump=None):
     """BASELINE config 4 at full size, STRONG-scaled: rank r owns a contiguous block of the prior draws; priors
     drawn on the device, 1e5-cell birth-death runs, distances + accept in the kernel epilogue, accepted draws
     packed into records on the device and all-gathered by the library (two ncclAllGather in one group).
-    The host waits once, before the simulation is enqueued (run_device fetches the 2 KB target distribution to
-    compute its statistics and CDF); simulation, packing and exchange then follow each other on the stream
-    without any host synchronisation up to the final event."""
+    The host waits once per pass, before the simulation is enqueued (run_device fetches the 2 KB target
+    distribution to compute its statistics and CDF); simulation, packing and exchange then follow each other on
+    the stream without any host synchronisation up to the final event.  `steps` timed passes over fresh prior
+    draws follow `warmup` untimed ones; `dump` is the --dump-outputs directory for the last timed pass."""
     m, torch, ctx = e.m, e.torch, e.ctx
     kw, _, desc = WORKLOADS["C4"]
     opts = m.SimulationOptions(save_snapshots=False, runs=draws_total, **kw)
@@ -525,25 +580,30 @@ def abc_leg(e, args, draws_total, with_cpu, with_e2e):
         marks[4].record()
 
     # warm-up: one pass at full size (every library buffer reaches its final size: no allocation in the timed
-    # pass), two reduced ones (kernels, the communicator)
-    for w in range(3):
+    # passes), then reduced ones (kernels, the communicator)
+    for w in range(warmup):
         one_pass(n if w == 0 else min(n, 32768), 500_000_000 + w * 2_000_000)
     barrier(e)
     sampler = ClockSampler(e.local_rank)
     sampler.start()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier(e)
+    events = 0
     e0.record()
-    one_pass(n, 0)
+    for s in range(steps):
+        if s:  # the previous pass's events (the next run_device waits for the stream anyway)
+            events += ctx.timing().total_events
+        one_pass(n, s * draws_total)
     e1.record()
     barrier(e)
     ms = e0.elapsed_time(e1)
     clocks = sampler.stop()
     tm = ctx.timing()
+    events += tm.total_events
     phases = {"priors_ms": marks[0].elapsed_time(marks[1]), "simulate_ms": marks[1].elapsed_time(marks[2]),
               "ssa_kernel_ms": tm.kernel_ms, "pack_ms": marks[2].elapsed_time(marks[3]),
               "allgather_ms": marks[3].elapsed_time(marks[4])}
-    ms_all, events_all = reduce_max_sum(e, ms, tm.total_events)
+    ms_all, events_all = reduce_max_sum(e, ms, events)
     counts = all_cnt_d.cpu().numpy().astype(np.int64)
     merged = m.merge_gathered(all_rec_d.cpu().numpy().view(np.uint32), counts, cap, ABC_BINS)
     rec = m.decode_records(merged, ABC_BINS)
@@ -552,21 +612,28 @@ def abc_leg(e, args, draws_total, with_cpu, with_e2e):
     ok = bool(len(rec["idx"]) == counts.sum() and np.all(np.diff(rec["idx"].astype(np.int64)) > 0) and
               counts[e.rank] == acc_local and np.all(rec["distance"][:, 0] <= ABC_THRESHOLDS[0]))
     post = rec["rates"][:, 1:].mean(axis=0).tolist() if len(rec["idx"]) else None
+    if dump:
+        dt = result_dtypes(m)
+        rows = {k: (v, dt[k]) for k, v in t.items()}
+        rows["prior_rates"] = (rates_d, np.float32)
+        dump_outputs(dump, rows, idx0 + (steps - 1) * draws_total, extra={"accepted_index": rec["idx"]},
+                     rank=e.rank, world=e.world)
 
     leg = Env()
     leg.kernel_ms, leg.alg_bytes, leg.events, leg.steps, leg.last = tm.kernel_ms, tm.alg_bytes, tm.total_events, 1, tm
-    out = {"metric": "abc_sims_per_sec", "value": draws_total / (ms_all * 1e-3), "unit": "sims/s", "n_gpus": e.world,
-           "scaling": "strong", "higher_is_better": True, "ms": ms_all, "events_per_sec": events_all / (ms_all * 1e-3),
+    out = {"metric": "abc_sims_per_sec", "value": draws_total * steps / (ms_all * 1e-3), "unit": "sims/s",
+           "n_gpus": e.world, "scaling": "strong", "higher_is_better": True, "steps": steps, "warmup": warmup,
+           "ms": ms_all / steps, "events_per_sec": events_all / (ms_all * 1e-3),
            "config": {"workload": f"C4: {desc}", "draws_total": draws_total, "draws_this_rank": n, "cells": opts.max_cells,
                       "thresholds": list(ABC_THRESHOLDS), "tile_width": tm.tile_width, "grid_blocks": tm.grid_blocks,
                       "record_words": words, "record_capacity_per_rank": cap,
                       "exchange": "ecdna_b200_abc_pack + ecdna_b200_abc_allgather (NCCL, 2 collectives in one group)"
                                   if e.world > 1 else "ecdna_b200_abc_pack (one rank: nothing to exchange)",
-                      "l2": "256 MiB buffer rewritten before the pass"},
+                      "l2": "256 MiB buffer rewritten before every pass"},
            "phases_this_rank": phases,
            "accepted_total": int(counts.sum()), "accepted_per_rank": counts.tolist(), "gather_ok": ok,
            "posterior_mean_b1_d0_d1": post, "stops_this_rank": stops.tolist(), "clocks": clocks,
-           "gpu_launches": tm.kernel_launches + 8, "roofline": roofline_block(leg, "C4", clocks)}
+           "gpu_launches": steps * (tm.kernel_launches + 8), "roofline": roofline_block(leg, "C4", clocks)}
 
     if with_e2e:
         # end to end through the host-buffer call: host prior draws in (16 B/draw), every draw's distances,
@@ -610,9 +677,11 @@ def main():
     m = e.m
 
     if args.workload == "C4":  # the ABC line on its own
-        a = abc_leg(e, args, args.abc_draws, not args.no_cpu_baseline, not args.no_e2e)
+        a = abc_leg(e, args, args.abc_draws, not args.no_cpu_baseline, not args.no_e2e, steps=args.steps,
+                    warmup=args.warmup, dump=args.dump_outputs)
         if rank == 0:
-            line = {"metric": a["metric"], "value": a["value"], "unit": a["unit"], "n_gpus": world, "steps": 1, "warmup": 3,
+            line = {"metric": a["metric"], "value": a["value"], "unit": a["unit"], "n_gpus": world, "steps": args.steps,
+                    "warmup": args.warmup,
                     "ms_per_step": a["ms"], "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
                     "dtype": "u32", "data": "synthetic"}
             line.update({k: v for k, v in a.items() if k not in line})
@@ -627,6 +696,11 @@ def main():
     check = {"C1": 3, "C2": 2, "C3": 4, "C5": 1}[args.workload]
     leg = ssa_leg(e, args, args.workload, reps, args.steps, args.warmup, opts0.idx_begin + rank * reps, check=check,
                   sample_clocks=True)
+    if args.dump_outputs:
+        dt = result_dtypes(m)
+        dump_outputs(args.dump_outputs, {k: (v, dt[k]) for k, v in leg.tensors.items()}, leg.last_idx0,
+                     rank=rank, world=world)
+    del leg.tensors
     e2e = None if args.no_e2e else e2e_ssa(e, leg, args.steps, opts0.idx_begin + 5_000_000_000 + rank * reps)
     roofline = roofline_block(leg, args.workload, leg.clocks)
 

@@ -57,51 +57,47 @@ class Out(C.Structure):
     ]
 
 
-_SO_FAST = os.path.join(_ORACLE_DIR, "libecdna_oracle_fast.so")
+_SOURCES = ("ecdna_oracle.cpp", "ecdna_oracle.h", "Makefile")
 
 
 def build(force=False):
-    src = [os.path.join(_ORACLE_DIR, f) for f in ("ecdna_oracle.cpp", "ecdna_oracle.h", "Makefile")]
-    stale = any((not os.path.exists(so)) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in src)
-                for so in (_SO, _SO_FAST))
+    """The checker, built in oracle/ when it is missing or older than its sources (__graft_entry__.build()
+    leaves it built, so a built tree is only read)."""
+    src = [os.path.join(_ORACLE_DIR, f) for f in _SOURCES]
+    stale = not os.path.exists(_SO) or any(os.path.getmtime(s) > os.path.getmtime(_SO) for s in src)
     if force or stale:
-        subprocess.run(["make", "-C", _ORACLE_DIR, "-B" if force else "-s"], check=True, capture_output=True)
+        subprocess.run(["make", "-s", "-C", _ORACLE_DIR] + (["-B"] if force else []) + ["libecdna_oracle.so"],
+                       check=True, capture_output=True)
     return _SO
 
 
 _lib = None
-_use_fast = False
-
-
-def _host_signature():
-    try:
-        for line in open("/proc/cpuinfo"):
-            if line.startswith("flags"):
-                import hashlib
-                return hashlib.sha256(line.encode()).hexdigest()
-    except OSError:
-        pass
-    return "unknown"
+_so_fast = None
 
 
 def use_fast_build():
     """bench.py's CPU legs time the -O3 -march=native build of the same source; tests never call this.
-    -march=native code must be compiled on the host that runs it: rebuilt when the CPU's flags differ."""
-    global _lib, _use_fast
-    if not _use_fast:
-        stamp = _SO_FAST + ".host"
-        sig = _host_signature()
-        if not os.path.exists(_SO_FAST) or not os.path.exists(stamp) or open(stamp).read().strip() != sig:
-            subprocess.run(["make", "-C", _ORACLE_DIR, "-B", "libecdna_oracle_fast.so"], check=True, capture_output=True)
-            open(stamp, "w").write(sig)
-        _use_fast, _lib = True, None
+    -march=native code must be compiled on the host that runs it, so it is compiled once per process, from a
+    copy of the sources in a temporary directory: the checkout may be read-only."""
+    global _lib, _so_fast
+    if _so_fast is None:
+        import atexit
+        import shutil
+        import tempfile
+        d = tempfile.mkdtemp(prefix="ecdna_oracle_fast_")
+        atexit.register(shutil.rmtree, d, True)
+        for f in _SOURCES:
+            shutil.copy(os.path.join(_ORACLE_DIR, f), d)
+        subprocess.run(["make", "-s", "-C", d, "libecdna_oracle_fast.so"], check=True, capture_output=True)
+        _so_fast, _lib = os.path.join(d, "libecdna_oracle_fast.so"), None
 
 
 def lib():
     global _lib
     if _lib is None:
-        build()
-        L = C.CDLL(_SO_FAST if _use_fast else _SO)
+        if _so_fast is None:
+            build()
+        L = C.CDLL(_so_fast or _SO)
         L.orc_run.argtypes = [C.POINTER(Opts), C.POINTER(Out)]
         L.orc_run.restype = C.c_int
         L.orc_run_batch.argtypes = [C.POINTER(Opts), C.c_uint64, C.c_uint64, C.c_int] + [C.c_void_p] * 6 + [
