@@ -17,8 +17,8 @@ import numpy as np
 
 from .build import LIB_PATH, build, build_debug  # noqa: F401
 from .shard import gather_accepted, rank_range  # noqa: F401
-from .abc import (ABC_FIELDS, REC_HEADER, abc_rows, decode_records, merge_gathered, record_words,  # noqa: F401
-                  write_abc_csv)
+from .abc import (ABC_FIELDS, REC_HEADER, SMC_FIELDS, abc_rows, decode_records, merge_gathered,  # noqa: F401
+                  record_words, write_abc_csv, write_abc_smc)
 
 ABI_VERSION = 3
 EV_BIRTH_NMINUS, EV_BIRTH_NPLUS, EV_DEATH_NMINUS, EV_DEATH_NPLUS = 0, 1, 2, 3
@@ -168,8 +168,30 @@ EXPORTED_SYMBOLS = [
     "ecdna_b200_multi_create", "ecdna_b200_multi_destroy", "ecdna_b200_multi_device_count",
     "ecdna_b200_multi_last_error", "ecdna_b200_multi_run", "ecdna_b200_multi_get_timing", "ecdna_b200_query_sizes",
     "ecdna_b200_run_sparse", "ecdna_b200_sparse_fetch", "ecdna_b200_multi_run_sparse", "ecdna_b200_multi_sparse_fetch",
+    "ecdna_b200_abc_smc_propose", "ecdna_b200_abc_smc_weights", "ecdna_b200_abc_smc",
 ]
 ERR_INTERNAL, ERR_COMM = 5, 6
+SMC_STATUS = ["reached", "max_generations", "budget"]  # ECDNA_B200_SMC_*
+
+
+class SmcOptionsT(C.Structure):
+    """ecdna_b200_smc_options_t"""
+    _fields_ = [("population", C.c_uint32), ("quantile", C.c_double), ("max_generations", C.c_uint32),
+                ("max_simulations", C.c_uint64), ("idx_begin", C.c_uint64), ("chunk", C.c_uint64),
+                ("b1_range", C.c_float * 2), ("d0_range", C.c_float * 2), ("d1_range", C.c_float * 2)]
+
+
+# (name, dtype, trailing shape) of the per-particle and per-generation outputs of ecdna_b200_smc_result_t
+SMC_PARTICLE_FIELDS = [("idx", np.uint64, ()), ("parent_idx", np.uint64, ()), ("rates", np.float32, (4,)),
+                       ("distance", np.float32, (4,)), ("weight", np.float64, ()), ("cells", np.uint64, ())]
+SMC_GENERATION_FIELDS = [("epsilon", np.float32, ()), ("consumed", np.uint64, ()), ("simulated", np.uint64, ()),
+                         ("ess", np.float64, ()), ("time_ms", np.float32, (3,))]
+
+
+class SmcResultT(C.Structure):
+    """ecdna_b200_smc_result_t"""
+    _fields_ = [(n, C.c_void_p) for n, _, _ in SMC_PARTICLE_FIELDS + SMC_GENERATION_FIELDS] + [
+        ("generations", C.c_uint32), ("status", C.c_uint32)]
 COMM_ID_BYTES = 128
 
 _lib = None
@@ -233,6 +255,12 @@ def lib():
         L.ecdna_b200_sparse_fetch.argtypes = [C.c_void_p, C.POINTER(SparseT)]
         L.ecdna_b200_multi_run_sparse.argtypes = L.ecdna_b200_run_sparse.argtypes
         L.ecdna_b200_multi_sparse_fetch.argtypes = [C.c_void_p, C.POINTER(SparseT)]
+        L.ecdna_b200_abc_smc_propose.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p,
+                                                 C.c_uint32, C.POINTER(C.c_double)] + [C.POINTER(C.c_float)] * 3 + [
+                                                     C.c_void_p, C.c_void_p]
+        L.ecdna_b200_abc_smc_weights.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32,
+                                                 C.POINTER(C.c_double)] + [C.POINTER(C.c_float)] * 3 + [C.c_void_p]
+        L.ecdna_b200_abc_smc.argtypes = [C.c_void_p, C.POINTER(ParamsT), C.POINTER(SmcOptionsT), C.POINTER(SmcResultT)]
         L.ecdna_b200_comm_release.argtypes = [C.c_void_p]
         L.ecdna_b200_comm_release.restype = None
         _lib = L
@@ -482,6 +510,34 @@ class Context:
                                                             C.c_void_p(rates_dev_ptr),
                                                             C.c_void_p(stream) if stream else None))
 
+    def abc_smc_propose(self, seed, idx_begin, n, prev_rates, cum_weights, sigma, b1_range=(1.0, 2.0),
+                        d0_range=(0.0, 0.5), d1_range=(0.0, 0.5)):
+        """ecdna_b200_abc_smc_propose: (rates [n][4] f32, parent [n] u32) of draws idx_begin .. idx_begin + n - 1,
+        proposed from the population prev_rates [M][4] with cumulative weights cum_weights [M] (f64)."""
+        prev = np.ascontiguousarray(prev_rates, dtype=np.float32).reshape(-1, 4)
+        cum = np.ascontiguousarray(cum_weights, dtype=np.float64)
+        assert len(cum) == len(prev)
+        rates, parent = np.zeros((n, 4), dtype=np.float32), np.zeros(n, dtype=np.uint32)
+        self._check(lib().ecdna_b200_abc_smc_propose(self._h, seed, idx_begin, n, prev.ctypes.data, cum.ctypes.data,
+                                                     len(prev), (C.c_double * 3)(*sigma), *_ranges(b1_range, d0_range,
+                                                                                                  d1_range),
+                                                     rates.ctypes.data, parent.ctypes.data))
+        return rates, parent
+
+    def abc_smc_weights(self, new_rates, prev_rates, prev_weights, sigma, b1_range=(1.0, 2.0), d0_range=(0.0, 0.5),
+                        d1_range=(0.0, 0.5)):
+        """ecdna_b200_abc_smc_weights: normalised importance weights [N] (f64) of new_rates [N][4] against the
+        population prev_rates [M][4] with weights prev_weights [M]."""
+        new = np.ascontiguousarray(new_rates, dtype=np.float32).reshape(-1, 4)
+        prev = np.ascontiguousarray(prev_rates, dtype=np.float32).reshape(-1, 4)
+        w = np.ascontiguousarray(prev_weights, dtype=np.float64)
+        assert len(w) == len(prev)
+        out = np.zeros(len(new), dtype=np.float64)
+        self._check(lib().ecdna_b200_abc_smc_weights(self._h, new.ctypes.data, len(new), prev.ctypes.data, w.ctypes.data,
+                                                     len(prev), (C.c_double * 3)(*sigma),
+                                                     *_ranges(b1_range, d0_range, d1_range), out.ctypes.data))
+        return out
+
     def abc_pack(self, results_struct, rates_dev_ptr, base_rates, idx_begin, n_runs, hist_stride, rec_bins, capacity,
                  records_dev_ptr, count_dev_ptr, stream=None):
         """ecdna_b200_abc_pack: accepted draws -> fixed-stride records on the device, in index order."""
@@ -542,6 +598,44 @@ class MultiContext(Context):
         t = TimingT()
         self._check(lib().ecdna_b200_multi_get_timing(self._h, C.byref(t)))
         return t
+
+    def abc_smc(self, opts, target, thresholds, population, quantile=0.5, max_generations=10,
+                max_simulations=10_000_000, b1_range=(1.0, 2.0), d0_range=(0.0, 0.5), d1_range=(0.0, 0.5), chunk=0,
+                idx_begin=None, **kw):
+        """ecdna_b200_abc_smc over the GPUs of this handle.  Returns a dict: the per-particle arrays of
+        SMC_PARTICLE_FIELDS as [generations][population][...], the per-generation arrays of SMC_GENERATION_FIELDS,
+        "generations", "status" (one of SMC_STATUS) and "options" (what write_abc_smc records)."""
+        idx_begin = opts.idx_begin if idx_begin is None else idx_begin
+        p = self.make_params(opts, 1, abc_target=np.ascontiguousarray(target, dtype=np.uint64),
+                             abc_thresholds=thresholds, snapshots=False, **kw)
+        o = SmcOptionsT()
+        o.population, o.quantile, o.max_generations = population, quantile, max_generations
+        o.max_simulations, o.idx_begin, o.chunk = max_simulations, idx_begin, chunk
+        o.b1_range[:], o.d0_range[:], o.d1_range[:] = b1_range, d0_range, d1_range
+        r = SmcResultT()
+        out = {}
+        G, M = max(int(max_generations), 1), max(int(population), 1)
+        for name, dtype, tail in SMC_PARTICLE_FIELDS:
+            out[name] = np.zeros((G, M) + tail, dtype=dtype)
+            setattr(r, name, out[name].ctypes.data)
+        for name, dtype, tail in SMC_GENERATION_FIELDS:
+            out[name] = np.zeros((G,) + tail, dtype=dtype)
+            setattr(r, name, out[name].ctypes.data)
+        self._check(lib().ecdna_b200_abc_smc(self._h, C.byref(p), C.byref(o), C.byref(r)))
+        g = int(r.generations)
+        out = {k: v[:g] for k, v in out.items()}
+        out["generations"], out["status"] = g, SMC_STATUS[r.status]
+        out["options"] = {"seed": int(opts.seed), "idx_begin": int(idx_begin), "population": int(population),
+                          "quantile": float(quantile), "max_generations": int(max_generations),
+                          "max_simulations": int(max_simulations), "b1_range": [float(np.float32(x)) for x in b1_range],
+                          "d0_range": [float(np.float32(x)) for x in d0_range],
+                          "d1_range": [float(np.float32(x)) for x in d1_range],
+                          "thresholds": [float(np.float32(x)) for x in thresholds]}
+        return out
+
+
+def _ranges(*ranges):
+    return [(C.c_float * 2)(*r) for r in ranges]
 
 
 def _addr(a):

@@ -1,9 +1,11 @@
 """ABC record writer: the CSV of the reference's removed `abc` binary (abc.md:38-55), one row per
-prior draw, ALL draws saved so the thresholds can be tuned afterwards (abc.md:57-71).
+prior draw, ALL draws saved so the thresholds can be tuned afterwards (abc.md:57-71); and the files of an
+ABC-SMC run, one CSV per generation's population plus abc_smc.json.
 
 Input is what the kernel's fused epilogue returns per draw (distances, accept flag, final counts) and
 the prior draws; nothing is simulated here."""
 import csv
+import os
 
 import numpy as np
 
@@ -68,3 +70,63 @@ def write_abc_csv(path, opts, idx_begin, rates, abc_distance, nminus, nplus, **k
             w.writerow(row)
             n += 1
     return n
+
+
+SMC_FIELDS = ABC_FIELDS + ["generation", "epsilon", "weight"]
+
+
+def _g9(x):
+    """printf("%.9g") of an f32 value: what `ecdna abc` writes (it round-trips f32)."""
+    return "%.9g" % float(x)
+
+
+def _g17(x):
+    """printf("%.17g") of an f64 value (round-trips f64)."""
+    return "%.17g" % float(x)
+
+
+def _cell(v):
+    return _g9(v) if isinstance(v, float) else str(v)
+
+
+def _json_float(s):
+    return {"inf": "Infinity", "-inf": "-Infinity"}.get(s, s)
+
+
+def write_abc_smc(path, opts, result):
+    """The files of an ABC-SMC run (MultiContext.abc_smc): <path>/abc_gen<t>.csv with generation t's population
+    (the columns of abc.md:38-55, parental_idx = the idx of the perturbed particle, then generation, epsilon,
+    weight) and <path>/abc_smc.json (per generation: epsilon, consumed and simulated draws, ESS; the status; the
+    options).  `ecdna abc --generations` writes the same bytes: f32 values as %.9g, f64 values as %.17g, "\n"
+    line ends.  Returns the number of generations written."""
+    os.makedirs(path, exist_ok=True)
+    G = int(result["generations"])
+    for t in range(G):
+        rates, dist, cells = result["rates"][t], result["distance"][t], result["cells"][t]
+        zeros = np.zeros(len(cells), dtype=np.uint64)
+        eps = _g9(result["epsilon"][t])
+        with open(os.path.join(path, f"abc_gen{t}.csv"), "w", newline="") as f:
+            f.write(",".join(SMC_FIELDS) + "\n")
+            for i, row in enumerate(abc_rows(opts, 0, rates, dist, cells, zeros)):
+                row["idx"] = int(result["idx"][t][i])
+                if t > 0:
+                    row["parental_idx"] = int(result["parent_idx"][t][i])
+                f.write(",".join(_cell(row[k]) for k in ABC_FIELDS) + f",{t},{eps},{_g17(result['weight'][t][i])}\n")
+    o = result["options"]
+
+    def arr(xs, fmt):
+        return "[" + ",".join(_json_float(fmt(x)) for x in xs) + "]"
+
+    opts_json = (f'{{"seed":{o["seed"]},"idx_begin":{o["idx_begin"]},"population":{o["population"]},'
+                 f'"quantile":{_g17(o["quantile"])},"max_generations":{o["max_generations"]},'
+                 f'"max_simulations":{o["max_simulations"]},"b1_range":{arr(o["b1_range"], _g9)},'
+                 f'"d0_range":{arr(o["d0_range"], _g9)},"d1_range":{arr(o["d1_range"], _g9)},'
+                 f'"thresholds":{arr(o["thresholds"], _g9)}}}')
+    text = (f'{{"status":"{result["status"]}","generations":{G},'
+            f'"epsilon":{arr(result["epsilon"][:G], _g9)},'
+            f'"consumed":[{",".join(str(int(x)) for x in result["consumed"][:G])}],'
+            f'"simulated":[{",".join(str(int(x)) for x in result["simulated"][:G])}],'
+            f'"ess":{arr(result["ess"][:G], _g17)},"options":{opts_json}}}\n')
+    with open(os.path.join(path, "abc_smc.json"), "w", newline="") as f:
+        f.write(text)
+    return G

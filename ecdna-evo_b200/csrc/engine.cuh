@@ -8,6 +8,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <string>
+#include <vector>
 
 #include "ssa_kernel.cuh"
 
@@ -61,7 +62,7 @@ struct ecdna_b200_ctx {
   std::string err;
   ecdna::DevBuf init_k, init_c, snap, rates, replay, replay_off, abc_cdf, arena, counters, scratch, park_list, park_rec,
       park_list2, park_rec2, order, order_hist, cells, zig, ts_ring, ts_rec, sub_sizes, hist_tmp, pack_idx, pack_out, pack_cnt,
-      sp_desc, sp_len, sp_bsum, sp_arena, cols[ecdna::C_COUNT];
+      sp_desc, sp_len, sp_bsum, sp_arena, smc_prev, smc_cum, smc_new, smc_parent, smc_tiles, smc_sum, cols[ecdna::C_COUNT];
   // the packed batch the last ecdna_b200_run_sparse left on the device (sparse.cuh)
   struct {
     bool valid = false, packed = false;
@@ -70,6 +71,16 @@ struct ecdna_b200_ctx {
   } sp;
   size_t arena_words = 0, arena_kcap = 0;
   ecdna_b200_timing_t timing{};
+};
+
+// several GPUs of one process (multi.cu); the ABC-SMC driver (abc_smc.cu) runs its proposals on the first one
+struct ecdna_b200_multi {
+  std::vector<ecdna_b200_ctx*> ctx;
+  std::vector<uint64_t> last_begin, last_count;
+  std::vector<uint64_t> sp_words;  // arena words of every GPU's block of the last sparse run
+  uint64_t sp_snap = 0, sp_sub = 0;
+  bool sp_valid = false;
+  std::string err;
 };
 
 namespace ecdna {

@@ -9,15 +9,6 @@
 
 using namespace ecdna;
 
-struct ecdna_b200_multi {
-  std::vector<ecdna_b200_ctx*> ctx;
-  std::vector<uint64_t> last_begin, last_count;
-  std::vector<uint64_t> sp_words;  // arena words of every GPU's block of the last sparse run
-  uint64_t sp_snap = 0, sp_sub = 0;
-  bool sp_valid = false;
-  std::string err;
-};
-
 namespace {
 // contiguous block of [0, n) owned by part r of `parts` (the first parts take the remainder)
 void block_of(uint64_t n, int r, int parts, uint64_t* begin, uint64_t* count) {

@@ -10,7 +10,8 @@
 // distributions come back as descriptors + occupied bins, a tenth of the dense form for the default snapshots),
 // in chunks, so that host memory is O(chunk) whatever --runs is; the files of a chunk are written while the
 // next one is simulated.  `ecdna abc --target FILE.json ...` is the front end of the reference's removed ABC
-// binary (abc.md:10-55): prior draws over (b1, d0, d1), one run per draw, abc.csv with every draw.
+// binary (abc.md:10-55): prior draws over (b1, d0, d1), one run per draw, abc.csv with every draw;
+// `ecdna abc --generations G` runs ABC-SMC instead (ecdna_b200_abc_smc) and writes one CSV per population.
 //
 // The reference is Rust; no Rust toolchain exists in this image, so the host side above the C ABI is
 // C++ (INTEGRATION.md shows the Rust binding a maintainer would add instead of this file).
@@ -66,6 +67,10 @@ struct Cli {
   std::string target;
   float b1_range[2] = {1.f, 2.f}, d0_range[2] = {0.f, 0.5f}, d1_range[2] = {0.f, 0.5f};
   float thresholds[4] = {0.05f, 0.1f, 0.1f, 0.1f};
+  // `ecdna abc --generations G`: ABC-SMC (0 = rejection ABC over --runs draws)
+  uint32_t generations = 0, population = 1000;
+  double quantile = 0.5;
+  uint64_t max_simulations = 10000000ull;
 };
 
 [[noreturn]] void die(const std::string& msg) {
@@ -105,7 +110,13 @@ void usage() {
       "  -h, --help\n  -V, --version\n\n"
       "ABC (abc.md): ecdna abc --target <FILE.json> [-r draws] [--b1-range lo,hi] [--d0-range lo,hi] [--d1-range lo,hi]\n"
       "              [--thresholds ks,mean,entropy,frequency] [--cells N] [--seed S] [--initial FILE] <DIR>\n"
-      "              writes <DIR>/abc.csv (every draw) and <DIR>/abc_accepted.csv");
+      "              writes <DIR>/abc.csv (every draw) and <DIR>/abc_accepted.csv\n"
+      "ABC-SMC:      ecdna abc --target <FILE.json> --generations <G> [--population M] [--quantile A]\n"
+      "              [--max-simulations S] [the ranges, thresholds and model options above] <DIR>\n"
+      "              populations of M particles [default: 1000], the tolerance of generation t+1 the A-quantile\n"
+      "              [default: 0.5] of generation t's distances, until the thresholds themselves are reached, G\n"
+      "              generations or S draws [default: 10000000]; writes <DIR>/abc_gen<t>.csv per generation and\n"
+      "              <DIR>/abc_smc.json (cannot be combined with --runs)");
 }
 
 std::vector<uint64_t> parse_list(const std::string& v) {
@@ -124,10 +135,16 @@ std::vector<uint64_t> parse_list(const std::string& v) {
 
 Cli parse(int argc, char** argv) {
   Cli c;
-  bool have_path = false, runs_given = false, verb_given = false;
+  bool have_path = false, runs_given = false, verb_given = false, smc_opt_given = false, generations_given = false;
   auto need = [&](int& i, const std::string& name) -> std::string {
     if (i + 1 >= argc) die("a value is required for '" + name + "' but none was supplied");
     return argv[++i];
+  };
+  auto number = [&](const std::string& v, const std::string& name) -> double {  // clap: "invalid value"
+    char* end = nullptr;
+    const double x = std::strtod(v.c_str(), &end);
+    if (v.empty() || *end) die("invalid value '" + v + "' for '" + name + "': invalid number");
+    return x;
   };
   auto pair_of = [&](const std::string& v, float* out) {
     const size_t comma = v.find(',');
@@ -183,6 +200,29 @@ Cli parse(int argc, char** argv) {
       while (std::getline(ss, tok, ',') && j < 4) c.thresholds[j++] = std::strtof(tok.c_str(), nullptr);
       if (j != 4) die("--thresholds needs four values: ks,mean,entropy,frequency");
     }
+    else if (a == "--generations") {
+      const double g = number(value(), "--generations <G>");
+      if (!(g >= 1.0 && g <= 4294967295.0) || g != std::floor(g)) die("invalid value for '--generations <G>': must be an integer >= 1");
+      c.generations = (uint32_t)g;
+      generations_given = true;
+    }
+    else if (c.abc && a == "--population") {
+      const double m = number(value(), "--population <M>");
+      if (!(m >= 1.0 && m <= 4294967295.0) || m != std::floor(m)) die("invalid value for '--population <M>': must be an integer >= 1");
+      c.population = (uint32_t)m;
+      smc_opt_given = true;
+    }
+    else if (c.abc && a == "--quantile") {
+      c.quantile = number(value(), "--quantile <A>");
+      if (!(c.quantile > 0.0 && c.quantile < 1.0)) die("invalid value for '--quantile <A>': must lie in (0, 1)");
+      smc_opt_given = true;
+    }
+    else if (c.abc && a == "--max-simulations") {
+      const double s = number(value(), "--max-simulations <S>");
+      if (!(s >= 0.0 && s < 1.8e19) || s != std::floor(s)) die("invalid value for '--max-simulations <S>': must be an integer >= 0 (0 = no limit)");
+      c.max_simulations = (uint64_t)s;
+      smc_opt_given = true;
+    }
     else if (a == "--tile-width") c.tile_width = (uint32_t)std::atoi(value().c_str());
     else if (a == "--state") {
       const std::string s = value();
@@ -196,6 +236,10 @@ Cli parse(int argc, char** argv) {
   }
   if (!have_path) die("the following required arguments were not provided:\n  <DIR>");
   if (c.abc && c.target.empty()) die("the following required arguments were not provided:\n  --target <FILE.json>");
+  if (generations_given && !c.abc) die("the argument '--generations <G>' is only valid after the 'abc' subcommand");
+  if (generations_given && runs_given) die("the argument '--generations <G>' cannot be used with '--runs <RUNS>'");
+  if (smc_opt_given && !generations_given)
+    die("the arguments '--population', '--quantile' and '--max-simulations' require '--generations <G>'");
   if (c.has_years && c.has_cells) die("the argument '--years <YEARS>' cannot be used with '--cells <CELLS>'");
   if (c.debug && (c.has_years || c.has_cells || c.sequential || runs_given || verb_given))
     die("the argument '--debug' cannot be used with one or more of the other specified arguments");
@@ -390,6 +434,94 @@ int run_abc(const Cli& c, ecdna_b200_multi* gpus, ecdna_b200_params_t p, uint64_
   return 0;
 }
 
+std::string g9(double v) {  // %.9g (round-trips f32); JSON spells infinity as Python's json module does
+  char buf[64];
+  std::snprintf(buf, sizeof buf, "%.9g", v);
+  return buf;
+}
+std::string g17(double v) {
+  char buf[64];
+  std::snprintf(buf, sizeof buf, "%.17g", v);
+  return buf;
+}
+std::string json_num(const std::string& s) { return s == "inf" ? "Infinity" : (s == "-inf" ? "-Infinity" : s); }
+
+// `ecdna abc --generations G`: ABC-SMC over the GPUs of `gpus` (ecdna_b200_abc_smc); <DIR>/abc_gen<t>.csv holds
+// population t in the columns of abc.csv (parental_idx = idx of the perturbed particle) plus generation, epsilon,
+// weight, and <DIR>/abc_smc.json the schedule.  Byte for byte what write_abc_smc (abc.py) writes for the same run.
+int run_abc_smc(const Cli& c, ecdna_b200_multi* gpus, ecdna_b200_params_t p, uint64_t idx_begin,
+                const std::map<uint32_t, uint64_t>& init) {
+  const std::map<uint32_t, uint64_t> tgt = load_json_hist(c.target);
+  std::vector<uint64_t> target((size_t)tgt.rbegin()->first + 1, 0);
+  for (auto& kv : tgt) target[kv.first] = kv.second;
+  uint64_t init_cells = 0, init_copies = 0;
+  for (auto& kv : init) { init_cells += kv.second; init_copies += (uint64_t)kv.first * kv.second; }
+  const double init_mean = init_cells ? (double)init_copies / (double)init_cells : 0.0;
+  p.abc_enabled = 1;
+  p.abc_target_hist = target.data();
+  p.abc_target_len = (uint32_t)target.size();
+  for (int j = 0; j < 4; ++j) p.abc_thresholds[j] = c.thresholds[j];
+  ecdna_b200_smc_options_t o;
+  std::memset(&o, 0, sizeof o);
+  o.population = c.population; o.quantile = c.quantile; o.max_generations = c.generations;
+  o.max_simulations = c.max_simulations; o.idx_begin = idx_begin; o.chunk = c.chunk;
+  for (int j = 0; j < 2; ++j) { o.b1_range[j] = c.b1_range[j]; o.d0_range[j] = c.d0_range[j]; o.d1_range[j] = c.d1_range[j]; }
+  const size_t G = c.generations, M = c.population;
+  std::vector<uint64_t> idx(G * M), parent(G * M), cells(G * M), consumed(G), simulated(G);
+  std::vector<float> rates(G * M * 4), dist(G * M * 4), eps(G);
+  std::vector<double> weight(G * M), ess(G);
+  ecdna_b200_smc_result_t r;
+  std::memset(&r, 0, sizeof r);
+  r.idx = idx.data(); r.parent_idx = parent.data(); r.rates = rates.data(); r.distance = dist.data();
+  r.weight = weight.data(); r.cells = cells.data(); r.epsilon = eps.data(); r.consumed = consumed.data();
+  r.simulated = simulated.data(); r.ess = ess.data();
+  const int rc = ecdna_b200_abc_smc(gpus, &p, &o, &r);
+  if (rc != ECDNA_B200_OK) { std::fprintf(stderr, "ecdna_b200_abc_smc: %s\n", ecdna_b200_multi_last_error(gpus)); return 101; }
+  mkdirs(c.path);
+  for (uint32_t t = 0; t < r.generations; ++t) {
+    const std::string file = c.path + "/abc_gen" + std::to_string(t) + ".csv";
+    std::ofstream f(file);
+    if (!f) { std::fprintf(stderr, "Cannot create %s\n", file.c_str()); return 101; }
+    f << "parental_idx,idx,timepoint,seed,ecdna,mean,entropy,f1,f2,d1,d2,cells,tumour_cells,init_mean,init_cells,init_copies,"
+         "generation,epsilon,weight\n";
+    const std::string e = g9(eps[t]);
+    for (size_t i = t * M; i < (t + 1) * M; ++i) {
+      const float* x = &rates[4 * i];
+      const float* d = &dist[4 * i];
+      // abc.md:44-52: f1/d1 belong to the cells WITH ecDNA, f2/d2 to the cells without
+      if (t > 0) f << parent[i];
+      f << "," << idx[i] << ",0," << c.seed << "," << g9(d[0]) << "," << g9(d[1]) << "," << g9(d[2]) << "," << g9(x[1]) << ","
+        << g9(x[0]) << "," << g9(x[3]) << "," << g9(x[2]) << "," << cells[i] << "," << cells[i] << "," << g9(init_mean) << ","
+        << init_cells << "," << init_copies << "," << t << "," << e << "," << g17(weight[i]) << "\n";
+    }
+  }
+  const char* status[] = {"reached", "max_generations", "budget"};
+  std::ofstream js(c.path + "/abc_smc.json");
+  if (!js) { std::fprintf(stderr, "Cannot create %s/abc_smc.json\n", c.path.c_str()); return 101; }
+  auto list = [&](auto n, auto fmt) {
+    std::string out = "[";
+    for (uint32_t t = 0; t < n; ++t) out += (t ? "," : "") + fmt(t);
+    return out + "]";
+  };
+  const uint32_t n = r.generations;
+  auto pair = [&](const float* v) { return "[" + g9(v[0]) + "," + g9(v[1]) + "]"; };
+  js << "{\"status\":\"" << status[r.status > 2 ? 2 : r.status] << "\",\"generations\":" << n
+     << ",\"epsilon\":" << list(n, [&](uint32_t t) { return json_num(g9(eps[t])); })
+     << ",\"consumed\":" << list(n, [&](uint32_t t) { return std::to_string(consumed[t]); })
+     << ",\"simulated\":" << list(n, [&](uint32_t t) { return std::to_string(simulated[t]); })
+     << ",\"ess\":" << list(n, [&](uint32_t t) { return json_num(g17(ess[t])); })
+     << ",\"options\":{\"seed\":" << c.seed << ",\"idx_begin\":" << idx_begin << ",\"population\":" << c.population
+     << ",\"quantile\":" << g17(c.quantile) << ",\"max_generations\":" << c.generations
+     << ",\"max_simulations\":" << c.max_simulations << ",\"b1_range\":" << pair(c.b1_range)
+     << ",\"d0_range\":" << pair(c.d0_range) << ",\"d1_range\":" << pair(c.d1_range) << ",\"thresholds\":"
+     << list(4u, [&](uint32_t j) { return json_num(g9(c.thresholds[j])); }) << "}}\n";
+  uint64_t total = 0;
+  for (uint32_t t = 0; t < n; ++t) total += simulated[t];
+  std::printf("%u generations (%s), %llu draws simulated, final tolerance factor %s\n", n, status[r.status > 2 ? 2 : r.status],
+              (unsigned long long)total, n ? g9(eps[n - 1]).c_str() : "-");
+  return 0;
+}
+
 }  // namespace
 
 int main(int argc, char** argv) {
@@ -456,7 +588,7 @@ int main(int argc, char** argv) {
   p.tile_width = c.tile_width; p.state_mode = c.state_mode;
   const uint64_t idx_begin = c.seed * 10;  // main.rs:214
   if (c.abc) {
-    const int arc = run_abc(c, gpus, p, idx_begin, runs, init);
+    const int arc = c.generations ? run_abc_smc(c, gpus, p, idx_begin, init) : run_abc(c, gpus, p, idx_begin, runs, init);
     ecdna_b200_multi_destroy(gpus);
     if (arc == 0) std::printf("%s End simulation\n", utc_now().c_str());
     return arc;

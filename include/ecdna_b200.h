@@ -358,6 +358,77 @@ int ecdna_b200_abc_allgather(ecdna_b200_ctx* ctx, const uint32_t* records_dev, c
                              uint32_t rec_bins, uint32_t capacity, uint32_t* all_records_dev,
                              uint32_t* all_counts_dev, void* cuda_stream);
 
+/* ---- ABC-SMC: sequential Monte Carlo ABC (ABC population Monte Carlo) over (b1, d0, d1) ----
+   Generation 0 is rejection ABC on the uniform prior box of ecdna_b200_abc_draw_priors: its first M valid draws.
+   Generation t+1 proposes from the weighted population t: a parent picked by weight, then every free parameter
+   perturbed by a Gaussian truncated to the box, sigma_k^2 = 2 x the weighted variance of parameter k in
+   population t (Beaumont, Cornuet, Marin, Robert 2009, Biometrika 96:983); its particles are weighted by
+   1 / sum_j W_j prod_k phi((theta_ik - theta_jk) / sigma_k) / Z_j with Z_j the truncation normaliser of parent j
+   (ibid.; the uniform prior cancels).  The tolerance eps (a factor on every user threshold thr_j > 0) follows the
+   quantile schedule eps_{t+1} = min(eps_t, max(1, rho_(ceil(alpha M)))) of the scalar distances
+   rho = max_j d_j / thr_j (Del Moral, Doucet, Jasra 2012, Stat. Comput. 22:1009) and the run ends after the first
+   generation at eps = 1, where acceptance is the rejection rule of the kernel's epilogue.  DESIGN.md section 9.
+   A range with lo == hi fixes that parameter: it is never perturbed and has no factor in the weights. */
+
+/* Proposals for draws idx_begin .. idx_begin + n - 1 (device kernel; host buffers in and out; blocking).
+   Draw i picks parent = the first j with cum_weights[j] > u * cum_weights[M-1] (u in [0,1), 53 bits of Philox
+   keyed (seed, i) in a domain of its own) and perturbs every free parameter k (lo < hi, sigma[k] > 0) by
+   z = Phi^-1(Phi(a) + u' (Phi(b) - Phi(a))), a, b = the box edges in sigma units around the parent, in f64;
+   no rejection loop.  prev_rates [M][4] (b0, b1, d0, d1), cum_weights [M] (f64, non-decreasing, last > 0),
+   rates_out [n][4] (column 0 and fixed parameters copied from the parent), parent_out [n] (0 .. M-1). */
+int ecdna_b200_abc_smc_propose(ecdna_b200_ctx* ctx, uint64_t seed, uint64_t idx_begin, uint64_t n,
+                               const float* prev_rates, const double* cum_weights, uint32_t M, const double sigma[3],
+                               const float b1_range[2], const float d0_range[2], const float d1_range[2],
+                               float* rates_out, uint32_t* parent_out);
+
+/* Importance weights of new_rates [N][4] against the population prev_rates [M][4] with weights prev_weights [M]
+   (f64) and kernel widths sigma[3]: all-pairs sum on the device in a fixed order (no atomics: bit-identical run to
+   run); weights_out [N] (f64) are normalised to sum to 1.  Host buffers; blocking. */
+int ecdna_b200_abc_smc_weights(ecdna_b200_ctx* ctx, const float* new_rates, uint32_t N, const float* prev_rates,
+                               const double* prev_weights, uint32_t M, const double sigma[3], const float b1_range[2],
+                               const float d0_range[2], const float d1_range[2], double* weights_out);
+
+enum { ECDNA_B200_SMC_REACHED = 0, ECDNA_B200_SMC_MAX_GENERATIONS = 1, ECDNA_B200_SMC_BUDGET = 2 };
+
+typedef struct {
+  uint32_t population;      /* M >= 1 particles per generation */
+  double quantile;          /* alpha in (0, 1): eps_{t+1} is the ceil(alpha M)-th smallest rho of generation t */
+  uint32_t max_generations; /* >= 1, generation 0 included */
+  uint64_t max_simulations; /* draw indices all generations may consume together; 0 = no limit */
+  uint64_t idx_begin;       /* index of the first draw (the CLI: seed * 10) */
+  uint64_t chunk;           /* draws per ecdna_b200_multi_run call; 0 = sized from the acceptance rate.
+                               Results do not depend on it (nor on the number of GPUs) */
+  float b1_range[2], d0_range[2], d1_range[2]; /* the uniform prior box, lo <= hi */
+} ecdna_b200_smc_options_t;
+
+/* Caller-owned; [G][M] below means [max_generations][population]; every pointer is optional (NULL = not wanted). */
+typedef struct {
+  uint64_t* idx;        /* [G][M] draw index of the particle (its SSA stream and its proposal stream) */
+  uint64_t* parent_idx; /* [G][M] draw index of the parent; UINT64_MAX in generation 0 */
+  float* rates;         /* [G][M][4] b0, b1, d0, d1 */
+  float* distance;      /* [G][M][4] ks, rel. mean, rel. entropy, rel. frequency */
+  double* weight;       /* [G][M] normalised importance weights */
+  uint64_t* cells;      /* [G][M] nminus + nplus at the end of the run */
+  float* epsilon;       /* [G] tolerance factor of the generation (+inf in generation 0) */
+  uint64_t* consumed;   /* [G] draw indices used: up to and including the M-th accepted draw */
+  uint64_t* simulated;  /* [G] draws simulated, including those past the M-th acceptance */
+  double* ess;          /* [G] effective sample size 1 / sum W_i^2 */
+  float* time_ms;       /* [G][3] host clock: simulation, proposal, weights */
+  uint32_t generations; /* out: generations completed */
+  uint32_t status;      /* out: ECDNA_B200_SMC_* */
+} ecdna_b200_smc_result_t;
+
+/* The ABC-SMC loop over every GPU of `m`.  params: b0, the process, the stop rule, the ABC target and the user
+   thresholds (abc_enabled set, at least one threshold >= 0, rates_per_run NULL); params->seed keys every stream.
+   Draw i is simulated as replicate i (its SSA stream is the one rejection ABC gives index i) through
+   ecdna_b200_multi_run in chunks; proposals and weights run on the first GPU.  A draw is accepted when the
+   epilogue accepts it at thresholds thr_j * eps (thr_j > 0; others unchanged) and it is valid: stop code neither
+   COPY_OVERFLOW nor HIST_OVERFLOW, no FLAG_HIST_TRUNCATED (copy numbers below params->hist_stride), finite rho.
+   Ends with status REACHED after the first generation at eps = 1, MAX_GENERATIONS, or BUDGET when the next
+   generation would pass max_simulations (the generations before it are returned; not an error). */
+int ecdna_b200_abc_smc(ecdna_b200_multi* m, const ecdna_b200_params_t* params, const ecdna_b200_smc_options_t* options,
+                       ecdna_b200_smc_result_t* result);
+
 #ifdef __cplusplus
 }
 #endif
