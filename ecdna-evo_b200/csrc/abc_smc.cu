@@ -188,9 +188,11 @@ int ecdna_b200_abc_smc_propose(ecdna_b200_ctx* ctx, uint64_t seed, uint64_t idx_
   CU(cudaMemcpyAsync(ctx->smc_prev.p, prev_rates, (size_t)M * 16, cudaMemcpyHostToDevice, st));
   CU(cudaMemcpyAsync(ctx->smc_cum.p, cum_weights, (size_t)M * 8, cudaMemcpyHostToDevice, st));
   const uint32_t n32 = (uint32_t)n;
-  smc_propose_kernel<<<(n32 + 255) / 256, 256, 0, st>>>((uint32_t)seed, (uint32_t)(seed >> 32), idx_begin, n32,
-                                                        (const float4*)ctx->smc_prev.p, (const double*)ctx->smc_cum.p, M,
-                                                        box, (float4*)ctx->smc_new.p, (uint32_t*)ctx->smc_parent.p);
+  // (grids in 64 bits: (n + 255) / 256 in 32 bits wraps to a few blocks for n > 2^32 - 256)
+  smc_propose_kernel<<<(uint32_t)((n + 255) / 256), 256, 0, st>>>((uint32_t)seed, (uint32_t)(seed >> 32), idx_begin,
+                                                                  n32, (const float4*)ctx->smc_prev.p,
+                                                                  (const double*)ctx->smc_cum.p, M, box,
+                                                                  (float4*)ctx->smc_new.p, (uint32_t*)ctx->smc_parent.p);
   CU(cudaGetLastError());
   CU(cudaMemcpyAsync(rates_out, ctx->smc_new.p, (size_t)n * 16, cudaMemcpyDeviceToHost, st));
   CU(cudaMemcpyAsync(parent_out, ctx->smc_parent.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
@@ -220,9 +222,10 @@ int ecdna_b200_abc_smc_weights(ecdna_b200_ctx* ctx, const float* new_rates, uint
   CU(cudaMemcpyAsync(ctx->smc_prev.p, prev_rates, (size_t)M * 16, cudaMemcpyHostToDevice, st));
   CU(cudaMemcpyAsync(ctx->smc_cum.p, prev_weights, (size_t)M * 8, cudaMemcpyHostToDevice, st));
   CU(cudaMemcpyAsync(ctx->smc_new.p, new_rates, (size_t)N * 16, cudaMemcpyHostToDevice, st));
-  smc_tiles_kernel<<<(M + 255) / 256, 256, 0, st>>>((const float4*)ctx->smc_prev.p, (const double*)ctx->smc_cum.p, M, box,
-                                                    (float4*)ctx->smc_tiles.p);
-  smc_pair_kernel<<<(N + kPairBlock - 1) / kPairBlock, kPairBlock, 0, st>>>(
+  smc_tiles_kernel<<<(uint32_t)(((uint64_t)M + 255) / 256), 256, 0, st>>>((const float4*)ctx->smc_prev.p,
+                                                                           (const double*)ctx->smc_cum.p, M, box,
+                                                                           (float4*)ctx->smc_tiles.p);
+  smc_pair_kernel<<<(uint32_t)(((uint64_t)N + kPairBlock - 1) / kPairBlock), kPairBlock, 0, st>>>(
       (const float4*)ctx->smc_new.p, N, (const float4*)ctx->smc_tiles.p, M, sc[0], sc[1], sc[2], (double*)ctx->smc_sum.p);
   CU(cudaGetLastError());
   CU(cudaMemcpyAsync(weights_out, ctx->smc_sum.p, (size_t)N * 8, cudaMemcpyDeviceToHost, st));

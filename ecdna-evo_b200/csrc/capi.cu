@@ -733,9 +733,10 @@ int ecdna_b200_abc_draw_priors(ecdna_b200_ctx* ctx, uint64_t seed, uint64_t idx_
   CU(cudaSetDevice(ctx->device));
   CU(ctx->rates.ensure(n_runs * 16));
   const uint32_t n = (uint32_t)n_runs;
-  prior_kernel<<<(n + 255) / 256, 256, 0, ctx->stream>>>((uint32_t)seed, (uint32_t)(seed >> 32), idx_begin, n, b0,
-                                                         b1_range[0], b1_range[1], d0_range[0], d0_range[1],
-                                                         d1_range[0], d1_range[1], (float*)ctx->rates.p);
+  // (the grid in 64 bits: (n + 255) / 256 in 32 bits wraps to a few blocks for n > 2^32 - 256)
+  prior_kernel<<<(uint32_t)((n_runs + 255) / 256), 256, 0, ctx->stream>>>(
+      (uint32_t)seed, (uint32_t)(seed >> 32), idx_begin, n, b0, b1_range[0], b1_range[1], d0_range[0], d0_range[1],
+      d1_range[0], d1_range[1], (float*)ctx->rates.p);
   CU(cudaGetLastError());
   CU(cudaMemcpyAsync(rates_out, ctx->rates.p, n_runs * 16, cudaMemcpyDeviceToHost, ctx->stream));
   CU(cudaStreamSynchronize(ctx->stream));
@@ -749,8 +750,9 @@ int ecdna_b200_abc_draw_priors_device(ecdna_b200_ctx* ctx, uint64_t seed, uint64
   CU(cudaSetDevice(ctx->device));
   const uint32_t n = (uint32_t)n_runs;
   cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
-  prior_kernel<<<(n + 255) / 256, 256, 0, st>>>((uint32_t)seed, (uint32_t)(seed >> 32), idx_begin, n, b0, b1_range[0],
-                                                b1_range[1], d0_range[0], d0_range[1], d1_range[0], d1_range[1], rates_dev);
+  prior_kernel<<<(uint32_t)((n_runs + 255) / 256), 256, 0, st>>>((uint32_t)seed, (uint32_t)(seed >> 32), idx_begin, n, b0,
+                                                                 b1_range[0], b1_range[1], d0_range[0], d0_range[1],
+                                                                 d1_range[0], d1_range[1], rates_dev);
   CU(cudaGetLastError());
   return ECDNA_B200_OK;
 }
