@@ -169,9 +169,11 @@ EXPORTED_SYMBOLS = [
     "ecdna_b200_multi_last_error", "ecdna_b200_multi_run", "ecdna_b200_multi_get_timing", "ecdna_b200_query_sizes",
     "ecdna_b200_run_sparse", "ecdna_b200_sparse_fetch", "ecdna_b200_multi_run_sparse", "ecdna_b200_multi_sparse_fetch",
     "ecdna_b200_abc_smc_propose", "ecdna_b200_abc_smc_weights", "ecdna_b200_abc_smc",
+    "ecdna_b200_abc_smc_propose_cov", "ecdna_b200_abc_smc_weights_cov", "ecdna_b200_abc_smc_ex",
 ]
 ERR_INTERNAL, ERR_COMM = 5, 6
 SMC_STATUS = ["reached", "max_generations", "budget"]  # ECDNA_B200_SMC_*
+SMC_KERNELS = ["component", "mvn", "olcm"]  # ECDNA_B200_SMC_KERNEL_*
 
 
 class SmcOptionsT(C.Structure):
@@ -186,6 +188,11 @@ SMC_PARTICLE_FIELDS = [("idx", np.uint64, ()), ("parent_idx", np.uint64, ()), ("
                        ("distance", np.float32, (4,)), ("weight", np.float64, ()), ("cells", np.uint64, ())]
 SMC_GENERATION_FIELDS = [("epsilon", np.float32, ()), ("consumed", np.uint64, ()), ("simulated", np.uint64, ()),
                          ("ess", np.float64, ()), ("time_ms", np.float32, (3,))]
+
+
+class SmcKernelT(C.Structure):
+    """ecdna_b200_smc_kernel_t"""
+    _fields_ = [("kernel", C.c_uint32), ("reserved", C.c_uint32 * 3)]
 
 
 class SmcResultT(C.Structure):
@@ -261,6 +268,14 @@ def lib():
         L.ecdna_b200_abc_smc_weights.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32,
                                                  C.POINTER(C.c_double)] + [C.POINTER(C.c_float)] * 3 + [C.c_void_p]
         L.ecdna_b200_abc_smc.argtypes = [C.c_void_p, C.POINTER(ParamsT), C.POINTER(SmcOptionsT), C.POINTER(SmcResultT)]
+        L.ecdna_b200_abc_smc_propose_cov.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p,
+                                                     C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32] + [
+                                                         C.POINTER(C.c_float)] * 3 + [C.c_void_p, C.c_void_p]
+        L.ecdna_b200_abc_smc_weights_cov.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p,
+                                                     C.c_uint32, C.c_void_p, C.c_uint32] + [
+                                                         C.POINTER(C.c_float)] * 3 + [C.c_void_p]
+        L.ecdna_b200_abc_smc_ex.argtypes = [C.c_void_p, C.POINTER(ParamsT), C.POINTER(SmcOptionsT),
+                                            C.POINTER(SmcKernelT), C.POINTER(SmcResultT), C.c_void_p]
         L.ecdna_b200_comm_release.argtypes = [C.c_void_p]
         L.ecdna_b200_comm_release.restype = None
         _lib = L
@@ -538,6 +553,36 @@ class Context:
                                                      *_ranges(b1_range, d0_range, d1_range), out.ctypes.data))
         return out
 
+    def abc_smc_propose_cov(self, seed, idx_begin, n, prev_rates, cum_weights, cov, b1_range=(1.0, 2.0),
+                            d0_range=(0.0, 0.5), d1_range=(0.0, 0.5)):
+        """ecdna_b200_abc_smc_propose_cov: as abc_smc_propose with the correlated kernel of cov, the packed lower
+        triangles (s11, s21, s22, s31, s32, s33) of one shared Sigma [6] or of one Sigma per parent [M][6]."""
+        prev = np.ascontiguousarray(prev_rates, dtype=np.float32).reshape(-1, 4)
+        cum = np.ascontiguousarray(cum_weights, dtype=np.float64)
+        cv = np.ascontiguousarray(cov, dtype=np.float64).reshape(-1, 6)
+        assert len(cum) == len(prev)
+        rates, parent = np.zeros((n, 4), dtype=np.float32), np.zeros(n, dtype=np.uint32)
+        self._check(lib().ecdna_b200_abc_smc_propose_cov(self._h, seed, idx_begin, n, prev.ctypes.data, cum.ctypes.data,
+                                                         len(prev), cv.ctypes.data, len(cv),
+                                                         *_ranges(b1_range, d0_range, d1_range), rates.ctypes.data,
+                                                         parent.ctypes.data))
+        return rates, parent
+
+    def abc_smc_weights_cov(self, new_rates, prev_rates, prev_weights, cov, b1_range=(1.0, 2.0), d0_range=(0.0, 0.5),
+                            d1_range=(0.0, 0.5)):
+        """ecdna_b200_abc_smc_weights_cov: normalised importance weights [N] (f64) of new_rates [N][4] under the
+        correlated kernels of cov ([6] or [M][6], as abc_smc_propose_cov) around prev_rates [M][4]."""
+        new = np.ascontiguousarray(new_rates, dtype=np.float32).reshape(-1, 4)
+        prev = np.ascontiguousarray(prev_rates, dtype=np.float32).reshape(-1, 4)
+        w = np.ascontiguousarray(prev_weights, dtype=np.float64)
+        cv = np.ascontiguousarray(cov, dtype=np.float64).reshape(-1, 6)
+        assert len(w) == len(prev)
+        out = np.zeros(len(new), dtype=np.float64)
+        self._check(lib().ecdna_b200_abc_smc_weights_cov(self._h, new.ctypes.data, len(new), prev.ctypes.data,
+                                                         w.ctypes.data, len(prev), cv.ctypes.data, len(cv),
+                                                         *_ranges(b1_range, d0_range, d1_range), out.ctypes.data))
+        return out
+
     def abc_pack(self, results_struct, rates_dev_ptr, base_rates, idx_begin, n_runs, hist_stride, rec_bins, capacity,
                  records_dev_ptr, count_dev_ptr, stream=None):
         """ecdna_b200_abc_pack: accepted draws -> fixed-stride records on the device, in index order."""
@@ -601,10 +646,14 @@ class MultiContext(Context):
 
     def abc_smc(self, opts, target, thresholds, population, quantile=0.5, max_generations=10,
                 max_simulations=10_000_000, b1_range=(1.0, 2.0), d0_range=(0.0, 0.5), d1_range=(0.0, 0.5), chunk=0,
-                idx_begin=None, **kw):
-        """ecdna_b200_abc_smc over the GPUs of this handle.  Returns a dict: the per-particle arrays of
-        SMC_PARTICLE_FIELDS as [generations][population][...], the per-generation arrays of SMC_GENERATION_FIELDS,
-        "generations", "status" (one of SMC_STATUS) and "options" (what write_abc_smc records)."""
+                idx_begin=None, kernel="component", **kw):
+        """ecdna_b200_abc_smc_ex over the GPUs of this handle with the perturbation kernel `kernel` (one of
+        SMC_KERNELS).  Returns a dict: the per-particle arrays of SMC_PARTICLE_FIELDS as [generations][population][...],
+        the per-generation arrays of SMC_GENERATION_FIELDS, "generations", "status" (one of SMC_STATUS), "kernel",
+        "kernel_used" (per generation: None for generation 0, else the kernel that ran after the fallback) and
+        "options" (what write_abc_smc records)."""
+        if kernel not in SMC_KERNELS:
+            raise ValueError(f"kernel must be one of {SMC_KERNELS}")
         idx_begin = opts.idx_begin if idx_begin is None else idx_begin
         p = self.make_params(opts, 1, abc_target=np.ascontiguousarray(target, dtype=np.uint64),
                              abc_thresholds=thresholds, snapshots=False, **kw)
@@ -621,10 +670,15 @@ class MultiContext(Context):
         for name, dtype, tail in SMC_GENERATION_FIELDS:
             out[name] = np.zeros((G,) + tail, dtype=dtype)
             setattr(r, name, out[name].ctypes.data)
-        self._check(lib().ecdna_b200_abc_smc(self._h, C.byref(p), C.byref(o), C.byref(r)))
+        used = np.zeros(G, dtype=np.uint32)
+        ker = SmcKernelT(SMC_KERNELS.index(kernel))
+        self._check(lib().ecdna_b200_abc_smc_ex(self._h, C.byref(p), C.byref(o), C.byref(ker), C.byref(r),
+                                                used.ctypes.data))
         g = int(r.generations)
         out = {k: v[:g] for k, v in out.items()}
         out["generations"], out["status"] = g, SMC_STATUS[r.status]
+        out["kernel"] = kernel
+        out["kernel_used"] = [None if u == 0xFFFFFFFF else SMC_KERNELS[u] for u in used[:g].tolist()]
         out["options"] = {"seed": int(opts.seed), "idx_begin": int(idx_begin), "population": int(population),
                           "quantile": float(quantile), "max_generations": int(max_generations),
                           "max_simulations": int(max_simulations), "b1_range": [float(np.float32(x)) for x in b1_range],

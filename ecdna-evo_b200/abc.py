@@ -93,12 +93,23 @@ def _json_float(s):
     return {"inf": "Infinity", "-inf": "-Infinity"}.get(s, s)
 
 
+def _kernel_json(result, G):
+    """'"kernel":...,"kernel_used":[...],' for the correlated kernels; nothing for the component kernel, whose files
+    stay those of a run without the choice."""
+    kernel = result.get("kernel", "component")
+    if kernel == "component":
+        return ""
+    used = ",".join("null" if k is None else f'"{k}"' for k in result["kernel_used"][:G])
+    return f'"kernel":"{kernel}","kernel_used":[{used}],'
+
+
 def write_abc_smc(path, opts, result):
     """The files of an ABC-SMC run (MultiContext.abc_smc): <path>/abc_gen<t>.csv with generation t's population
     (the columns of abc.md:38-55, parental_idx = the idx of the perturbed particle, then generation, epsilon,
     weight) and <path>/abc_smc.json (per generation: epsilon, consumed and simulated draws, ESS; the status; the
-    options).  `ecdna abc --generations` writes the same bytes: f32 values as %.9g, f64 values as %.17g, "\n"
-    line ends.  Returns the number of generations written."""
+    options; with the mvn or olcm kernel also the kernel and the one each generation used).  `ecdna abc
+    --generations` writes the same bytes: f32 values as %.9g, f64 values as %.17g, "\n" line ends.  Returns the
+    number of generations written."""
     os.makedirs(path, exist_ok=True)
     G = int(result["generations"])
     for t in range(G):
@@ -126,7 +137,7 @@ def write_abc_smc(path, opts, result):
             f'"epsilon":{arr(result["epsilon"][:G], _g9)},'
             f'"consumed":[{",".join(str(int(x)) for x in result["consumed"][:G])}],'
             f'"simulated":[{",".join(str(int(x)) for x in result["simulated"][:G])}],'
-            f'"ess":{arr(result["ess"][:G], _g17)},"options":{opts_json}}}\n')
+            f'"ess":{arr(result["ess"][:G], _g17)},{_kernel_json(result, G)}"options":{opts_json}}}\n')
     with open(os.path.join(path, "abc_smc.json"), "w", newline="") as f:
         f.write(text)
     return G

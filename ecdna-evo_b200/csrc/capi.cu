@@ -680,7 +680,7 @@ void ecdna_b200_destroy(ecdna_b200_ctx* ctx) {
                     &ctx->abc_cdf, &ctx->arena, &ctx->counters, &ctx->scratch, &ctx->park_list, &ctx->park_rec, &ctx->park_list2, &ctx->park_rec2, &ctx->order, &ctx->order_hist, &ctx->ts_ring, &ctx->ts_rec, &ctx->sub_sizes, &ctx->hist_tmp,
                     &ctx->cells, &ctx->zig, &ctx->pack_idx, &ctx->pack_out, &ctx->pack_cnt, &ctx->sp_desc, &ctx->sp_len,
                     &ctx->sp_bsum, &ctx->sp_arena, &ctx->smc_prev, &ctx->smc_cum, &ctx->smc_new, &ctx->smc_parent,
-                    &ctx->smc_tiles, &ctx->smc_sum};
+                    &ctx->smc_tiles, &ctx->smc_sum, &ctx->smc_cov};
   for (DevBuf* b : bufs) b->release();
   for (auto& b : ctx->cols) b.release();
   cudaEventDestroy(ctx->ev_begin); cudaEventDestroy(ctx->ev_k0); cudaEventDestroy(ctx->ev_k1); cudaEventDestroy(ctx->ev_end);

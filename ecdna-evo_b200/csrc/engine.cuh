@@ -62,7 +62,8 @@ struct ecdna_b200_ctx {
   std::string err;
   ecdna::DevBuf init_k, init_c, snap, rates, replay, replay_off, abc_cdf, arena, counters, scratch, park_list, park_rec,
       park_list2, park_rec2, order, order_hist, cells, zig, ts_ring, ts_rec, sub_sizes, hist_tmp, pack_idx, pack_out, pack_cnt,
-      sp_desc, sp_len, sp_bsum, sp_arena, smc_prev, smc_cum, smc_new, smc_parent, smc_tiles, smc_sum, cols[ecdna::C_COUNT];
+      sp_desc, sp_len, sp_bsum, sp_arena, smc_prev, smc_cum, smc_new, smc_parent, smc_tiles, smc_sum, smc_cov,
+      cols[ecdna::C_COUNT];
   // the packed batch the last ecdna_b200_run_sparse left on the device (sparse.cuh)
   struct {
     bool valid = false, packed = false;

@@ -11,7 +11,7 @@
 // in chunks, so that host memory is O(chunk) whatever --runs is; the files of a chunk are written while the
 // next one is simulated.  `ecdna abc --target FILE.json ...` is the front end of the reference's removed ABC
 // binary (abc.md:10-55): prior draws over (b1, d0, d1), one run per draw, abc.csv with every draw;
-// `ecdna abc --generations G` runs ABC-SMC instead (ecdna_b200_abc_smc) and writes one CSV per population.
+// `ecdna abc --generations G` runs ABC-SMC instead (ecdna_b200_abc_smc_ex) and writes one CSV per population.
 //
 // The reference is Rust; no Rust toolchain exists in this image, so the host side above the C ABI is
 // C++ (INTEGRATION.md shows the Rust binding a maintainer would add instead of this file).
@@ -71,6 +71,7 @@ struct Cli {
   uint32_t generations = 0, population = 1000;
   double quantile = 0.5;
   uint64_t max_simulations = 10000000ull;
+  uint32_t smc_kernel = ECDNA_B200_SMC_KERNEL_COMPONENT;
 };
 
 [[noreturn]] void die(const std::string& msg) {
@@ -112,11 +113,13 @@ void usage() {
       "              [--thresholds ks,mean,entropy,frequency] [--cells N] [--seed S] [--initial FILE] <DIR>\n"
       "              writes <DIR>/abc.csv (every draw) and <DIR>/abc_accepted.csv\n"
       "ABC-SMC:      ecdna abc --target <FILE.json> --generations <G> [--population M] [--quantile A]\n"
-      "              [--max-simulations S] [the ranges, thresholds and model options above] <DIR>\n"
+      "              [--max-simulations S] [--kernel K] [the ranges, thresholds and model options above] <DIR>\n"
       "              populations of M particles [default: 1000], the tolerance of generation t+1 the A-quantile\n"
       "              [default: 0.5] of generation t's distances, until the thresholds themselves are reached, G\n"
       "              generations or S draws [default: 10000000]; writes <DIR>/abc_gen<t>.csv per generation and\n"
-      "              <DIR>/abc_smc.json (cannot be combined with --runs)");
+      "              <DIR>/abc_smc.json (cannot be combined with --runs); --kernel: the perturbation kernel\n"
+      "              [default: component] [possible values: component (a Gaussian per parameter), mvn (2 x the\n"
+      "              population covariance), olcm (a local covariance per particle)]");
 }
 
 std::vector<uint64_t> parse_list(const std::string& v) {
@@ -223,6 +226,14 @@ Cli parse(int argc, char** argv) {
       c.max_simulations = (uint64_t)s;
       smc_opt_given = true;
     }
+    else if (c.abc && a == "--kernel") {
+      const std::string v = value();
+      if (v == "component") c.smc_kernel = ECDNA_B200_SMC_KERNEL_COMPONENT;
+      else if (v == "mvn") c.smc_kernel = ECDNA_B200_SMC_KERNEL_MVN;
+      else if (v == "olcm") c.smc_kernel = ECDNA_B200_SMC_KERNEL_OLCM;
+      else die("invalid value '" + v + "' for '--kernel' [possible values: component, mvn, olcm]");
+      smc_opt_given = true;
+    }
     else if (a == "--tile-width") c.tile_width = (uint32_t)std::atoi(value().c_str());
     else if (a == "--state") {
       const std::string s = value();
@@ -239,7 +250,7 @@ Cli parse(int argc, char** argv) {
   if (generations_given && !c.abc) die("the argument '--generations <G>' is only valid after the 'abc' subcommand");
   if (generations_given && runs_given) die("the argument '--generations <G>' cannot be used with '--runs <RUNS>'");
   if (smc_opt_given && !generations_given)
-    die("the arguments '--population', '--quantile' and '--max-simulations' require '--generations <G>'");
+    die("the arguments '--population', '--quantile', '--max-simulations' and '--kernel' require '--generations <G>'");
   if (c.has_years && c.has_cells) die("the argument '--years <YEARS>' cannot be used with '--cells <CELLS>'");
   if (c.debug && (c.has_years || c.has_cells || c.sequential || runs_given || verb_given))
     die("the argument '--debug' cannot be used with one or more of the other specified arguments");
@@ -446,7 +457,7 @@ std::string g17(double v) {
 }
 std::string json_num(const std::string& s) { return s == "inf" ? "Infinity" : (s == "-inf" ? "-Infinity" : s); }
 
-// `ecdna abc --generations G`: ABC-SMC over the GPUs of `gpus` (ecdna_b200_abc_smc); <DIR>/abc_gen<t>.csv holds
+// `ecdna abc --generations G`: ABC-SMC over the GPUs of `gpus` (ecdna_b200_abc_smc_ex); <DIR>/abc_gen<t>.csv holds
 // population t in the columns of abc.csv (parental_idx = idx of the perturbed particle) plus generation, epsilon,
 // weight, and <DIR>/abc_smc.json the schedule.  Byte for byte what write_abc_smc (abc.py) writes for the same run.
 int run_abc_smc(const Cli& c, ecdna_b200_multi* gpus, ecdna_b200_params_t p, uint64_t idx_begin,
@@ -475,8 +486,12 @@ int run_abc_smc(const Cli& c, ecdna_b200_multi* gpus, ecdna_b200_params_t p, uin
   r.idx = idx.data(); r.parent_idx = parent.data(); r.rates = rates.data(); r.distance = dist.data();
   r.weight = weight.data(); r.cells = cells.data(); r.epsilon = eps.data(); r.consumed = consumed.data();
   r.simulated = simulated.data(); r.ess = ess.data();
-  const int rc = ecdna_b200_abc_smc(gpus, &p, &o, &r);
-  if (rc != ECDNA_B200_OK) { std::fprintf(stderr, "ecdna_b200_abc_smc: %s\n", ecdna_b200_multi_last_error(gpus)); return 101; }
+  ecdna_b200_smc_kernel_t kernel;
+  std::memset(&kernel, 0, sizeof kernel);
+  kernel.kernel = c.smc_kernel;
+  std::vector<uint32_t> used(G);
+  const int rc = ecdna_b200_abc_smc_ex(gpus, &p, &o, &kernel, &r, used.data());
+  if (rc != ECDNA_B200_OK) { std::fprintf(stderr, "ecdna_b200_abc_smc_ex: %s\n", ecdna_b200_multi_last_error(gpus)); return 101; }
   mkdirs(c.path);
   for (uint32_t t = 0; t < r.generations; ++t) {
     const std::string file = c.path + "/abc_gen" + std::to_string(t) + ".csv";
@@ -509,8 +524,13 @@ int run_abc_smc(const Cli& c, ecdna_b200_multi* gpus, ecdna_b200_params_t p, uin
      << ",\"epsilon\":" << list(n, [&](uint32_t t) { return json_num(g9(eps[t])); })
      << ",\"consumed\":" << list(n, [&](uint32_t t) { return std::to_string(consumed[t]); })
      << ",\"simulated\":" << list(n, [&](uint32_t t) { return std::to_string(simulated[t]); })
-     << ",\"ess\":" << list(n, [&](uint32_t t) { return json_num(g17(ess[t])); })
-     << ",\"options\":{\"seed\":" << c.seed << ",\"idx_begin\":" << idx_begin << ",\"population\":" << c.population
+     << ",\"ess\":" << list(n, [&](uint32_t t) { return json_num(g17(ess[t])); });
+  const char* kernels[] = {"component", "mvn", "olcm"};
+  if (c.smc_kernel != ECDNA_B200_SMC_KERNEL_COMPONENT)  // (the component kernel's files stay those of a run without it)
+    js << ",\"kernel\":\"" << kernels[c.smc_kernel] << "\",\"kernel_used\":" << list(n, [&](uint32_t t) {
+      return used[t] > 2 ? std::string("null") : "\"" + std::string(kernels[used[t]]) + "\"";
+    });
+  js << ",\"options\":{\"seed\":" << c.seed << ",\"idx_begin\":" << idx_begin << ",\"population\":" << c.population
      << ",\"quantile\":" << g17(c.quantile) << ",\"max_generations\":" << c.generations
      << ",\"max_simulations\":" << c.max_simulations << ",\"b1_range\":" << pair(c.b1_range)
      << ",\"d0_range\":" << pair(c.d0_range) << ",\"d1_range\":" << pair(c.d1_range) << ",\"thresholds\":"

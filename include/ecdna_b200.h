@@ -429,6 +429,45 @@ typedef struct {
 int ecdna_b200_abc_smc(ecdna_b200_multi* m, const ecdna_b200_params_t* params, const ecdna_b200_smc_options_t* options,
                        ecdna_b200_smc_result_t* result);
 
+/* ---- ABC-SMC with correlated perturbation kernels (DESIGN.md section 9) ----
+   COMPONENT: the kernel above (one Gaussian per parameter).  MVN: N(theta_j, Sigma), Sigma = 2 x the weighted
+   covariance of the population.  OLCM (Filippi, Barnes, Cornebise, Stumpf 2013, SAGMB 12:87): N(theta_j, Sigma_j),
+   Sigma_j = C + (m - theta_j)(m - theta_j)^T, m and C the weighted mean and covariance of the particles with
+   rho <= eps_{t+1}.  Both are truncated to the box by sequential conditioning over the free parameters in the order
+   b1, d0, d1 with L = chol(Sigma) (f64): coordinate t is N(c_t + sum_{l<t} L_tl e_l, L_tt^2) truncated to [lo, hi]
+   by inverse CDF (in log space beyond 5 sds), e_t = (theta_t - its mean) / L_tt; no rejection loop.  The density
+   prod_t phi(e_t) / (L_tt (Phi(b_t) - Phi(a_t))) with e = L^-1 (theta - c) is exact.  Draw i uses the Philox
+   words of ecdna_b200_abc_smc_propose, so a diagonal Sigma gives its proposals bit for bit. */
+enum { ECDNA_B200_SMC_KERNEL_COMPONENT = 0, ECDNA_B200_SMC_KERNEL_MVN = 1, ECDNA_B200_SMC_KERNEL_OLCM = 2 };
+
+/* cov: packed lower triangles (s11, s21, s22, s31, s32, s33) over (b1, d0, d1), f64; n_cov = 1 (shared) or M (one
+   per parent).  A parameter is free when lo < hi and its variance is > 0 in every Sigma (0 in every Sigma fixes it;
+   anything else is an error).  Rows/columns of fixed parameters are ignored; a non-finite entry or a Sigma that is
+   not positive definite over the free ones -> ERR_BAD_PARAMS.  Otherwise as ecdna_b200_abc_smc_propose. */
+int ecdna_b200_abc_smc_propose_cov(ecdna_b200_ctx* ctx, uint64_t seed, uint64_t idx_begin, uint64_t n,
+                                   const float* prev_rates, const double* cum_weights, uint32_t M, const double* cov,
+                                   uint32_t n_cov, const float b1_range[2], const float d0_range[2],
+                                   const float d1_range[2], float* rates_out, uint32_t* parent_out);
+
+/* Importance weights of new_rates [N][4] under the kernels of ecdna_b200_abc_smc_propose_cov: all-pairs sum in a
+   fixed order as ecdna_b200_abc_smc_weights (bit-identical run to run); weights_out [N] normalised to sum to 1. */
+int ecdna_b200_abc_smc_weights_cov(ecdna_b200_ctx* ctx, const float* new_rates, uint32_t N, const float* prev_rates,
+                                   const double* prev_weights, uint32_t M, const double* cov, uint32_t n_cov,
+                                   const float b1_range[2], const float d0_range[2], const float d1_range[2],
+                                   double* weights_out);
+
+typedef struct {
+  uint32_t kernel;      /* ECDNA_B200_SMC_KERNEL_* */
+  uint32_t reserved[3]; /* 0 */
+} ecdna_b200_smc_kernel_t;
+
+/* ecdna_b200_abc_smc with a choice of kernel (NULL = COMPONENT, which is ecdna_b200_abc_smc byte for byte).  Sigma is
+   usable when every Cholesky pivot L_tt >= 2^-12 (hi_t - lo_t); each generation falls back OLCM -> MVN -> COMPONENT
+   to the first usable one.  kernel_used [max_generations], optional: UINT32_MAX for generation 0, else the
+   ECDNA_B200_SMC_KERNEL_* that proposed and weighted the generation. */
+int ecdna_b200_abc_smc_ex(ecdna_b200_multi* m, const ecdna_b200_params_t* params, const ecdna_b200_smc_options_t* options,
+                          const ecdna_b200_smc_kernel_t* kernel, ecdna_b200_smc_result_t* result, uint32_t* kernel_used);
+
 #ifdef __cplusplus
 }
 #endif

@@ -3,10 +3,12 @@ target one run at (1.4, 0.2, 0.2), thresholds 0.05/0.1/0.1/0.1 times each of --s
 <out>/abc_smc_compare.json, per threshold scale:
 
 - rejection ABC: draws and device time until the M-th accepted draw (or the acceptance rate over --rejection-max);
-- ABC-SMC with population M: per generation epsilon, consumed and simulated draws, ESS, and the host-clock time of
-  the simulation, proposal and weight steps;
-- the weight kernel alone at N = M = --pairs-n: call time (host clock around the blocking call, copies included) and
-  kernel time (torch.profiler, a run of its own), pair evaluations per second.
+- ABC-SMC with population M, once per perturbation kernel of --kernels (component, mvn, olcm): per generation
+  epsilon, consumed and simulated draws, ESS, the kernel each generation used, and the host-clock time of the
+  simulation, proposal and weight steps; the totals, the posterior means and the final population's weighted
+  correlation matrix ("smc" for the component kernel, "smc_<kernel>" for the others);
+- the weight kernel of each of --kernels alone at N = M = --pairs-n: call time (host clock around the blocking call,
+  copies included) and pair-kernel time (torch.profiler, a run of its own), pair evaluations per second.
 
 The card's name and power limit are read in the same run.  Usage: python scripts/abc_smc_compare.py OUT_DIR"""
 import argparse
@@ -56,7 +58,9 @@ def main():
     ap.add_argument("--rejection-chunk", type=int, default=250_000)
     ap.add_argument("--pairs-n", type=int, default=100_000)
     ap.add_argument("--scales", default="1,0.5,0.25,0.125", help="factors on C4's thresholds, one comparison each")
+    ap.add_argument("--kernels", default="component", help="perturbation kernels to run: component,mvn,olcm")
     a = ap.parse_args()
+    kernels = a.kernels.split(",")
     os.makedirs(a.out, exist_ok=True)
     import _pkg
     m = _pkg.load()
@@ -92,24 +96,31 @@ def main():
                                "note": "device time covers every simulated chunk (CUDA events)"}
         print(json.dumps(entry["rejection"]), flush=True)
 
-        # ---- ABC-SMC to the same thresholds ----
-        t0 = time.perf_counter()
-        r = mc.abc_smc(opts, target, thr, M, quantile=a.quantile, max_generations=a.max_generations,
-                       max_simulations=a.max_simulations, **BOX)
-        wall = time.perf_counter() - t0
-        g = r["generations"]
-        entry["smc"] = {"status": r["status"], "generations": g, "epsilon": [float(x) for x in r["epsilon"]],
-                         "consumed": [int(x) for x in r["consumed"]], "simulated": [int(x) for x in r["simulated"]],
-                         "ess": [float(x) for x in r["ess"]],
-                         "ms_simulation": [float(x) for x in r["time_ms"][:, 0]],
-                         "ms_proposal": [float(x) for x in r["time_ms"][:, 1]],
-                         "ms_weights": [float(x) for x in r["time_ms"][:, 2]],
-                         "total_simulated": int(r["simulated"].sum()), "total_consumed": int(r["consumed"].sum()),
-                         "wall_s": wall}
-        if g:
-            w, th = r["weight"][-1], r["rates"][-1][:, 1:].astype(np.float64)
-            entry["smc"]["posterior_mean_b1_d0_d1"] = [float(np.sum(w * th[:, k])) for k in range(3)]
-        print(json.dumps(entry["smc"]), flush=True)
+        # ---- ABC-SMC to the same thresholds, with each kernel ----
+        for kernel in kernels:
+            t0 = time.perf_counter()
+            r = mc.abc_smc(opts, target, thr, M, quantile=a.quantile, max_generations=a.max_generations,
+                           max_simulations=a.max_simulations, kernel=kernel, **BOX)
+            wall = time.perf_counter() - t0
+            g = r["generations"]
+            e = {"kernel": kernel, "status": r["status"], "generations": g, "epsilon": [float(x) for x in r["epsilon"]],
+                 "consumed": [int(x) for x in r["consumed"]], "simulated": [int(x) for x in r["simulated"]],
+                 "ess": [float(x) for x in r["ess"]], "kernel_used": r["kernel_used"],
+                 "ms_simulation": [float(x) for x in r["time_ms"][:, 0]],
+                 "ms_proposal": [float(x) for x in r["time_ms"][:, 1]],
+                 "ms_weights": [float(x) for x in r["time_ms"][:, 2]],
+                 "total_simulated": int(r["simulated"].sum()), "total_consumed": int(r["consumed"].sum()),
+                 "wall_s": wall}
+            if g:
+                w, th = r["weight"][-1], r["rates"][-1][:, 1:].astype(np.float64)
+                mean = w @ th
+                cov = (w[:, None] * (th - mean)).T @ (th - mean)
+                sd = np.sqrt(np.diag(cov))
+                e["posterior_mean_b1_d0_d1"] = [float(x) for x in mean]
+                e["posterior_sd_b1_d0_d1"] = [float(x) for x in sd]
+                e["posterior_corr"] = (cov / np.outer(sd, sd)).tolist()
+            entry["smc" if kernel == "component" else f"smc_{kernel}"] = e
+            print(json.dumps(e), flush=True)
     mc.close()
 
     # ---- the weight kernel alone ----
@@ -120,31 +131,43 @@ def main():
         return np.column_stack([np.ones(N), rng.uniform(1, 2, N), rng.uniform(0, 0.5, (N, 2))]).astype(np.float32)
     new, prev = particles(), particles()
     w = np.full(N, 1.0 / N)
+    th = prev[:, 1:].astype(np.float64)
     sigma = tuple(float(np.sqrt(2 * prev[:, k].var())) for k in (1, 2, 3))
-    ctx.abc_smc_weights(new, prev, w, sigma, **BOX)  # warm-up: module load, buffers
-    times = []
-    for _ in range(5):
-        t0 = time.perf_counter()
-        ctx.abc_smc_weights(new, prev, w, sigma, **BOX)
-        times.append((time.perf_counter() - t0) * 1e3)
-    kernel = None
-    try:
-        import torch
-        from torch.profiler import ProfilerActivity, profile
-        with profile(activities=[ProfilerActivity.CUDA]) as prof:
-            for _ in range(3):
-                ctx.abc_smc_weights(new, prev, w, sigma, **BOX)
-            torch.cuda.synchronize()
-        ks = [e.device_time for e in prof.events() if "smc_pair_kernel" in e.name]
-        kernel = float(np.median(ks)) / 1e3 if ks else None  # ms
-    except Exception as e:  # the call times above stand on their own
-        print(f"profiler: {e}", file=sys.stderr)
-    pairs = float(N) * N
-    report["weights_kernel"] = {"N": N, "M": N, "call_ms_median": float(np.median(times)), "call_ms_all": times,
-                                "pair_kernel_ms": kernel,
-                                "pairs_per_s_call": pairs / (np.median(times) / 1e3),
-                                "pairs_per_s_kernel": pairs / (kernel / 1e3) if kernel else None}
-    print(json.dumps(report["weights_kernel"]), flush=True)
+    S = 2.0 * np.cov(th.T, bias=True)
+    tri = [(0, 0), (1, 0), (1, 1), (2, 0), (2, 1), (2, 2)]
+    mvn = np.array([S[r, c] for r, c in tri])
+    v = th.mean(axis=0) - th  # OLCM with every particle selected: Sigma_j = Cov + v_j v_j^T
+    olcm = np.stack([S[r, c] / 2 + v[:, r] * v[:, c] for r, c in tri], axis=1)
+    calls = {"component": (lambda: ctx.abc_smc_weights(new, prev, w, sigma, **BOX), "smc_pair_kernel"),
+             "mvn": (lambda: ctx.abc_smc_weights_cov(new, prev, w, mvn, **BOX), "smc_pair_cov_kernel<true>"),
+             "olcm": (lambda: ctx.abc_smc_weights_cov(new, prev, w, olcm, **BOX), "smc_pair_cov_kernel<false>")}
+    report["weights_kernel"] = {}
+    for kernel in kernels:
+        call, name = calls[kernel]
+        call()  # warm-up: module load, buffers
+        times = []
+        for _ in range(5):
+            t0 = time.perf_counter()
+            call()
+            times.append((time.perf_counter() - t0) * 1e3)
+        kms = None
+        try:
+            import torch
+            from torch.profiler import ProfilerActivity, profile
+            with profile(activities=[ProfilerActivity.CUDA]) as prof:
+                for _ in range(3):
+                    call()
+                torch.cuda.synchronize()
+            ks = [e.device_time for e in prof.events() if name in e.name.replace(" ", "")]
+            kms = float(np.median(ks)) / 1e3 if ks else None  # ms
+        except Exception as e:  # the call times above stand on their own
+            print(f"profiler: {e}", file=sys.stderr)
+        pairs = float(N) * N
+        rec = {"N": N, "M": N, "call_ms_median": float(np.median(times)), "call_ms_all": times,
+               "pair_kernel_ms": kms, "pairs_per_s_call": pairs / (np.median(times) / 1e3),
+               "pairs_per_s_kernel": pairs / (kms / 1e3) if kms else None}
+        report["weights_kernel"][kernel] = rec
+        print(kernel, json.dumps(rec), flush=True)
     ctx.close()
     with open(os.path.join(a.out, "abc_smc_compare.json"), "w") as f:
         json.dump(report, f, indent=1)
