@@ -144,7 +144,7 @@ void target_stats(const std::vector<uint64_t>& h, float* mean, float* ent, float
   unsigned long long eq = 0;  // (the same fixed-point entropy as the device epilogue: bit-identical)
   uint64_t cum = 0;
   for (size_t k = 0; k < h.size(); ++k) {
-    if (h[k]) eq += entropy_term_q40((float)h[k] / nf);
+    if (h[k]) eq += entropy_term_q40(h[k], n);
     cum += h[k];
     (*cdf)[k] = (float)cum / nf;
   }

@@ -434,16 +434,22 @@ void dense_hist(uint64_t* dst, uint32_t cap, uint64_t nminus, HistFn&& each) {
   each([&](uint32_t k, uint64_t c) { if (k < cap) dst[k] += c; });
 }
 
-// One term of the entropy, -p log2(p) for 0 < p <= 1, as a 2^-40 fixed-point integer: single IEEE f32 operations
-// in a fixed order (the polynomial of neg_log_u24 on the mantissa of p), so that the sum - an integer - does
-// not depend on the order of the terms.  The kernel's epilogue computes the same bits.
-inline uint64_t entropy_term_q40(float p) {
+// One term of the entropy, -p log2(p) for p = c / n, 0 < c <= n < 2^32, as a 2^-40 fixed-point integer: single
+// IEEE f32 operations in a fixed order (the polynomial of neg_log_u24 on the mantissa of p = f32(c) / f32(n)), so
+// that the sum - an integer - does not depend on the order of the terms.  A class that holds at least 3/4 of the
+// cells gives the polynomial x = p - 1 = -f32(n - c) / f32(n) directly, which keeps 1 - p when it is small.  The
+// kernel's epilogue computes the same bits.
+inline uint64_t entropy_term_q40(uint64_t c, uint64_t n) {
+  const float nf = (float)n;
+  const bool near1 = 4 * c >= 3 * n;
+  const float q = (float)(near1 ? n - c : c) / nf;  // 1 - p or p
+  const float p = near1 ? 1.0f - q : q;
   uint32_t bits; std::memcpy(&bits, &p, 4);
   int e = (int)(bits >> 23) - 127;
   uint32_t fb = (bits & 0x007FFFFFu) | 0x3F800000u;
   float f; std::memcpy(&f, &fb, 4);
   if (f > 1.41421356f) { f = f * 0.5f; e += 1; }
-  const float x = f - 1.0f;
+  const float x = near1 ? -q : f - 1.0f;  // (p in [3/4, 1]: its mantissa reduces to p itself, e = 0)
   const float z = x * x;
   float y = 7.0376836292E-2f;
   y = fmaf(y, x, -1.1514610310E-1f);
@@ -464,6 +470,16 @@ inline uint64_t entropy_term_q40(float p) {
   return (uint64_t)(std::fmax(t, 0.0f) * 1099511627776.0f);
 }
 
+// (n s2 - s1^2) / n^2 from the exact moments (n < 2^32): the numerator exact in 128 bits, rounded once to f64
+// (an FMA of its 48-bit halves), two f64 divisions by n, one rounding to f32.  The kernel's epilogue computes the
+// same bits.
+inline float variance_from_moments(uint64_t n, uint64_t s1, uint64_t s2) {
+  const unsigned __int128 d = (unsigned __int128)n * s2 - (unsigned __int128)s1 * s1;
+  const double hi = (double)(uint64_t)(d >> 48), lo = (double)(uint64_t)(d & 0xFFFFFFFFFFFFull);
+  const double nd = (double)n;
+  return (float)(std::fma(hi, 281474976710656.0, lo) / nd / nd);
+}
+
 void stats_from_dense(const uint64_t* hist, uint32_t cap, float* mean, float* freq, float* entropy, float* variance) {
   // ecdna-lib 3.0.2 summary statistics [RECALL R8]: all cells counted, zeros included; entropy in bits
   uint64_t n = 0, s1 = 0, s2 = 0;
@@ -473,11 +489,11 @@ void stats_from_dense(const uint64_t* hist, uint32_t cap, float* mean, float* fr
   const float mu = (float)s1 / nf;
   uint64_t eq = 0;
   for (uint32_t k = 0; k < cap; ++k)
-    if (hist[k]) eq += entropy_term_q40((float)hist[k] / nf);
+    if (hist[k]) eq += entropy_term_q40(hist[k], n);
   *mean = mu;
   *freq = (float)(n - hist[0]) / nf;
   *entropy = (float)eq * 9.094947017729282e-13f;  // 2^-40
-  *variance = (float)s2 / nf - mu * mu;
+  *variance = variance_from_moments(n, s1, s2);
 }
 
 template <class State> struct StateOps;
